@@ -13,6 +13,11 @@ buffers for b and x.  The matrix (871 MB) is far larger than L2 (126 MB), so
 every iteration streams it from HBM: no explicit L2 flush is needed.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload poisson215]
+                    [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed solve returned to its caller as DIR/<name>.npy (see
+dump_outputs), so that two builds can be compared output for output on identical inputs.  It is refused for
+--impl reference and for multi-rank runs (--gpus N > 1 under torchrun): only the single-GPU timed path dumps.
 """
 from __future__ import annotations
 
@@ -38,6 +43,7 @@ WORKLOADS = {
     "poisson32": (32, 79),        # BASELINE config 1  (CPU-runnable reference case)
 }
 FALLBACK_HBM_GBS = 6650.0         # B200_PROFILING.md fallback when MEASURED_PEAKS.json is absent
+DUMP_SAMPLE = 1 << 21             # entries of x written by --dump-outputs: 16 MB of values + 16 MB of positions
 
 
 def workload_name(N, iters):
@@ -223,6 +229,24 @@ def device_random_csr(torch, dev, n, per_row=20, seed=1234, shift=3.0):
     return rp.to(torch.int32), ci, out
 
 
+def dump_outputs(out_dir, x, stats):
+    """Writes what one solve returned to its caller, in float64: x.npy (the solution; above DUMP_SAMPLE entries a
+    fixed, seeded stratified sample of it), x_index.npy (the positions of those entries), niter.npy and solved.npy.
+    The timed solve keeps no residual history, so there are no residual norms to write.  The strata split [0, n)
+    into DUMP_SAMPLE contiguous ranges that cover it to the last entry, and one seeded position is drawn from each."""
+    import torch
+    n = int(x.numel())
+    if n > DUMP_SAMPLE:
+        bounds = np.arange(DUMP_SAMPLE + 1, dtype=np.int64) * n // DUMP_SAMPLE
+        idx = bounds[:-1] + np.random.default_rng(0).integers(0, np.diff(bounds))
+    else:
+        idx = np.arange(n, dtype=np.int64)
+    xs = x[torch.from_numpy(idx).to(x.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("x", xs), ("x_index", idx), ("niter", [stats.niter]), ("solved", [stats.solved])):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def extra_records(kb, torch, dev, peak):
     """BASELINE configs 3 and 4 on the same GPU (it/s + fraction of their own algorithmic-byte roofline,
     SURVEY.md 8d).  Not the headline metric: reported under "extra" on the N = 1 line."""
@@ -361,7 +385,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg and the parity block")
     ap.add_argument("--no-extra", action="store_true", help="skip the cfg3 / cfg4 extra records")
     ap.add_argument("--no-cfg5", dest="no_cfg5", action="store_true", help="skip the cfg5 (n ~ 1e8) record")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed solve returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl == "reference" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs is supported for the single-process GPU run (--impl ours, one rank)")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -394,7 +423,6 @@ def main():
     solve_kw = dict(atol=0.0, rtol=0.0, itmax=iters)
     for _ in range(args.warmup):
         ws.solve(None, b, **solve_kw)
-    assert ws.stats.niter == iters, ws.stats
     sampler = ClockSampler(local)
     sampler.start()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -407,6 +435,9 @@ def main():
     torch.cuda.synchronize()
     clocks = sampler.stop()
     launches = ws.launches - l0
+    assert ws.stats.niter == iters, ws.stats
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ws.x, ws.stats)
     ms = e0.elapsed_time(e1)
     its = args.steps * iters
     value = its / (ms * 1e-3)

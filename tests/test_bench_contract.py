@@ -78,3 +78,48 @@ def test_bench_helpers_on_cpu():
     assert g["ok"] and g["iters_compared"] == bench.WORKLOADS["poisson464"][1]
     assert bench.golden_parity([1.0, 2.0], "no_such_file")["ok"] is None
     assert bench.algorithmic_bytes_cg(215 ** 3, 7 * 215 ** 3 - 6 * 215 ** 2) == 1586811804        # SURVEY.md 8(d)
+
+
+def test_dump_outputs_writes_a_fixed_sample_of_the_solution(tmp_path):
+    """--dump-outputs: non-empty float64 .npy files, under 64 MB in all, and the same seeded positions from run to run
+    so that two builds can be compared entry by entry."""
+    import types
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    n = 3 * bench.DUMP_SAMPLE + 7
+    x = torch.arange(n, dtype=torch.float64) * 0.5
+    stats = types.SimpleNamespace(niter=200, solved=False)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), x, stats)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["niter.npy", "solved.npy", "x.npy", "x_index.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 << 20
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float64 and a.size > 0 and np.array_equal(a, b), f
+    idx, xs = np.load(tmp_path / "a" / "x_index.npy"), np.load(tmp_path / "a" / "x.npy")
+    assert len(idx) == bench.DUMP_SAMPLE and np.all(np.diff(idx) > 0) and 0 <= idx[0] and idx[-1] < n
+    k = np.arange(bench.DUMP_SAMPLE)
+    lo, hi = k * n // bench.DUMP_SAMPLE, (k + 1) * n // bench.DUMP_SAMPLE
+    assert np.all((lo <= idx) & (idx < hi))                          # one position per stratum, the last ending at n
+    assert idx[-1] >= n - (n + bench.DUMP_SAMPLE - 1) // bench.DUMP_SAMPLE
+    assert np.array_equal(xs, idx * 0.5)
+    assert np.load(tmp_path / "a" / "niter.npy").tolist() == [200.0]
+    small = torch.ones(10, dtype=torch.float64)
+    bench.dump_outputs(str(tmp_path / "c"), small, types.SimpleNamespace(niter=3, solved=True))
+    assert np.array_equal(np.load(tmp_path / "c" / "x.npy"), np.ones(10))
+    assert np.load(tmp_path / "c" / "solved.npy").tolist() == [1.0]
+
+
+@pytest.mark.parametrize("argv,env", [(["--steps", "0"], {}), (["--warmup", "-1"], {}),
+                                      (["--impl", "reference", "--dump-outputs", "d"], {}),
+                                      (["--dump-outputs", "d"], {"WORLD_SIZE": "2"})])
+def test_bench_rejects_bad_arguments(argv, env, tmp_path):
+    """A step count below 1, a negative warm-up, and --dump-outputs outside the single-GPU timed path are usage
+    errors (exit 2) raised before any work starts, and nothing is written."""
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True,
+                         timeout=120, cwd=tmp_path, env=dict(os.environ, **env))
+    assert out.returncode == 2 and "error:" in out.stderr and not out.stdout, (out.returncode, out.stderr[-500:])
+    assert not os.listdir(tmp_path)
