@@ -142,6 +142,10 @@ int krylov_b200_set_operator_csr(void *ws, int n, long long nnz, const void *row
 int krylov_b200_share_operator(void *ws, void *src);
 /* Attach a CSR object made by kb200_csr_create (not owned: keep it alive while `ws` uses it). */
 int krylov_b200_attach_csr(void *ws, void *csr);
+/* How the staged SpMV and the persistent CG kernel stream the attached CSR operator: the number of entries of its
+ * (column - row, value) dictionary when it is stored as one code byte per nonzero, 0 when they stream the CSR
+ * arrays (more than 256 distinct pairs, a non-default tile plan, or KB200_CSR_DICT=0 at upload), -1 on error. */
+int krylov_b200_operator_encoding(void *ws);
 /* Diagonal preconditioner: which = 0 -> M, 1 -> N; d[n] holds the diagonal of
  * the operator the solver applies (P^-1 with the default ldiv=false). NULL detaches. */
 int krylov_b200_set_preconditioner_diag(void *ws, int which, const void *d, int location);

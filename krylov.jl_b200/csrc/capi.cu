@@ -578,6 +578,13 @@ int krylov_b200_attach_csr(void* ws, void* csr) {
   return 0;
 }
 
+int krylov_b200_operator_encoding(void* ws) {
+  Handle* h = lookup_any(ws);
+  if (!h) return fail("krylov_b200_operator_encoding", "unknown workspace handle");
+  if (!h->csr) return fail("krylov_b200_operator_encoding", "no CSR operator attached");
+  return h->dtype == KRYLOV_FLOAT64 ? h->csr->d.ndict : h->csr->f.ndict;
+}
+
 int krylov_b200_set_preconditioner_diag(void* ws, int which, const void* d, int location) {
   try {
     Handle* h = lookup_any(ws);

@@ -442,7 +442,8 @@ __device__ __forceinline__ void cg_stage_halo(HaloMap halo, const CgPeerTab<T>* 
   }
 }
 
-template <class T, int MODE, int MINB, int DEPTH>
+// DICT: the matrix streams as the operator's dictionary codes (Csr::code); kPlain and kJacobi at 3 CTAs per SM.
+template <class T, int MODE, int MINB, int DEPTH, bool DICT>
 __global__ void __launch_bounds__(kTileThreads, MINB) cg_persist(Csr<T> A, CgPersistArgs<T> a, CgState<T>* st, T* part,
                                                                 GridBar* gb, DistComm* dc) {
   extern __shared__ __align__(128) unsigned char smem[];
@@ -452,7 +453,7 @@ __global__ void __launch_bounds__(kTileThreads, MINB) cg_persist(Csr<T> A, CgPer
   volatile CgState<T>* vst = st;
   if (vst->done) { cg_report_to_host<T>(a, st); return; }    // uniform: st only changes inside the barriers below
   if (threadIdx.x == 0) cg_load_scal<T>(st, &sc);            // published by the __syncthreads of P.init below
-  TilePipe<T> P;
+  TilePipe<T, DICT> P;
   P.init(A, smem);
   const int G = gridDim.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int cnt = (A.ntiles - (int)blockIdx.x + G - 1) / G;         // grid <= ntiles: cnt >= 1
@@ -481,7 +482,7 @@ __global__ void __launch_bounds__(kTileThreads, MINB) cg_persist(Csr<T> A, CgPer
     if (warp == kConsumerWarps) {
       if (lane == 0) {
         const unsigned target = (unsigned)(k + 1) * (unsigned)cnt + (k + 1 < a.max_iters ? pre : 0u);
-        tile_issue_until<T>(A, P, ppos, target, cnt, tile_at, pol);
+        tile_issue_until<T, DICT>(A, P, ppos, target, cnt, tile_at, pol);
       }
     } else {
       const T* r = MODE == kBlockJac ? a.z : a.r;      // block-Jacobi: gather z = M r (materialised by phase B)
@@ -513,14 +514,14 @@ __global__ void __launch_bounds__(kTileThreads, MINB) cg_persist(Csr<T> A, CgPer
         if (lane == 0) atomicAdd(&gb->halo_ready, 1u);       // 8 consumer warps per CTA report
         // interior tiles first; the tiles with halo columns (last in this CTA's sequence) only after every CTA's
         // producer warp has staged its share of the halo
-        tile_consume_pass<T, DEPTH>(A, P, cpos, 0, cnt_int, tile_at, gather, row_begin, row_done);
+        tile_consume_pass<T, DEPTH, DICT>(A, P, cpos, 0, cnt_int, tile_at, gather, row_begin, row_done);
         if (cnt_int < cnt) {
           if (lane == 0) { while (ld_acquire_gpu_u32(&gb->halo_ready) < (unsigned)(G * kConsumerWarps)) { } }
           __syncwarp();
-          tile_consume_pass<T, DEPTH>(A, P, cpos, cnt_int, cnt, tile_at, gather, row_begin, row_done);
+          tile_consume_pass<T, DEPTH, DICT>(A, P, cpos, cnt_int, cnt, tile_at, gather, row_begin, row_done);
         }
       } else {
-        tile_consume_pass<T, DEPTH>(A, P, cpos, 0, cnt, tile_at, gather, row_begin, row_done);
+        tile_consume_pass<T, DEPTH, DICT>(A, P, cpos, 0, cnt, tile_at, gather, row_begin, row_done);
       }
     }
     passes = k + 1;
@@ -583,7 +584,7 @@ __global__ void __launch_bounds__(kTileThreads, MINB) cg_persist(Csr<T> A, CgPer
       if (!ok || sc.done) break;
     }
   }
-  if (warp == kConsumerWarps && lane == 0) tile_drain<T>(P, (unsigned)passes * (unsigned)cnt, ppos);
+  if (warp == kConsumerWarps && lane == 0) tile_drain<T, DICT>(P, (unsigned)passes * (unsigned)cnt, ppos);
   cg_report_to_host<T>(a, st);                 // st is final: every CTA left the loop after the same barrier
 }
 
@@ -788,6 +789,7 @@ void cg_fused_loop(Workspace<T>& ws, const Csr<T>& A, const SolveOpts& o, T gamm
   typedef void (*KpFn)(Csr<T>, CgPersistArgs<T>, CgState<T>*, T*, GridBar*, DistComm*);
   KpFn kp = nullptr;
   int pgrid = 0;
+  size_t psmem = 0;
   CgPersistArgs<T> pa;
   memset(&pa, 0, sizeof(pa));
   GridBar* gbar = (GridBar*)((char*)ws.fused_state + kOffGridBar);
@@ -796,19 +798,26 @@ void cg_fused_loop(Workspace<T>& ws, const Csr<T>& A, const SolveOpts& o, T gamm
     // loads of an 8-nonzero gather batch in flight per thread; selected with KB200_CTAS_PER_SM=2 / large tiles)
     static const char* edep = getenv("KB200_GATHER_DEPTH");
     const int depth = edep ? atoi(edep) : 0;
-    if (A.ctas_per_sm >= 3) {
+    // The dictionary-encoded operator streams ~1 byte per nonzero instead of 12 (DESIGN.md section 3); the plan only
+    // builds it for the default 3-CTA/SM ring, and the encoded kernel runs the same grid, so the dot-product trees and
+    // with them every iterate are those of the CSR kernel.
+    const bool dict = A.ndict > 0 && !dist && !bjac && depth != 4;
+    if (dict) {
+      kp = jac ? cg_persist<T, kJacobi, 3, 8, true> : cg_persist<T, kPlain, 3, 8, true>;
+    } else if (A.ctas_per_sm >= 3) {
       // measured on cfg2 (profiles/README.md, round 2): 8-deep batches 3825 it/s, 4-deep 3691 it/s
-      if (bjac) kp = cg_persist<T, kBlockJac, 2, 8>;   // the block code of phase B needs the 96-register budget (2 CTAs per SM)
-      else if (depth == 4) kp = dist ? cg_persist<T, kDist, 3, 4> : (jac ? cg_persist<T, kJacobi, 3, 4> : cg_persist<T, kPlain, 3, 4>);
-      else kp = dist ? cg_persist<T, kDist, 3, 8> : (jac ? cg_persist<T, kJacobi, 3, 8> : cg_persist<T, kPlain, 3, 8>);
+      if (bjac) kp = cg_persist<T, kBlockJac, 2, 8, false>;   // the block code of phase B needs the 96-register budget (2 CTAs per SM)
+      else if (depth == 4) kp = dist ? cg_persist<T, kDist, 3, 4, false> : (jac ? cg_persist<T, kJacobi, 3, 4, false> : cg_persist<T, kPlain, 3, 4, false>);
+      else kp = dist ? cg_persist<T, kDist, 3, 8, false> : (jac ? cg_persist<T, kJacobi, 3, 8, false> : cg_persist<T, kPlain, 3, 8, false>);
     } else {
-      if (bjac) kp = cg_persist<T, kBlockJac, 2, 8>;
-      else if (depth == 4) kp = dist ? cg_persist<T, kDist, 2, 4> : (jac ? cg_persist<T, kJacobi, 2, 4> : cg_persist<T, kPlain, 2, 4>);
-      else kp = dist ? cg_persist<T, kDist, 2, 8> : (jac ? cg_persist<T, kJacobi, 2, 8> : cg_persist<T, kPlain, 2, 8>);
+      if (bjac) kp = cg_persist<T, kBlockJac, 2, 8, false>;
+      else if (depth == 4) kp = dist ? cg_persist<T, kDist, 2, 4, false> : (jac ? cg_persist<T, kJacobi, 2, 4, false> : cg_persist<T, kPlain, 2, 4, false>);
+      else kp = dist ? cg_persist<T, kDist, 2, 8, false> : (jac ? cg_persist<T, kJacobi, 2, 8, false> : cg_persist<T, kPlain, 2, 8, false>);
     }
+    psmem = dict ? A.dict_smem_bytes : A.smem_bytes;
     ensure_dyn_smem((const void*)kp, 220 * 1024);
     int occ = 0;
-    KB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kp, kTileThreads, A.smem_bytes));
+    KB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kp, kTileThreads, psmem));
     if (occ < 1) throw std::runtime_error("cg_persist does not fit on an SM with the planned shared-memory ring");
     pgrid = std::min(std::min(occ, A.ctas_per_sm) * sm_count(), std::max(1, A.ntiles));
     pa.r = ws.r; pa.P0 = ws.p; pa.P1 = ws.p2; pa.Ap = ws.Ap; pa.x = ws.x;
@@ -872,7 +881,7 @@ void cg_fused_loop(Workspace<T>& ws, const Csr<T>& A, const SolveOpts& o, T gamm
       pa.hseq = hseq + slot;
       pa.seq = expect[slot] = ++ws.fused_seq;
       void* args[] = {(void*)&Acopy, (void*)&pa, (void*)&dst, (void*)&partp, (void*)&gbar, (void*)&dcm};
-      KB_CUDA(cudaLaunchCooperativeKernel((const void*)kp, dim3(pgrid), dim3(kTileThreads), args, A.smem_bytes, c.stream));
+      KB_CUDA(cudaLaunchCooperativeKernel((const void*)kp, dim3(pgrid), dim3(kTileThreads), args, psmem, c.stream));
       c.launches += 1;
       enq += batch;
       return;                                   // the kernel reports into pinned host memory itself

@@ -96,7 +96,16 @@ struct Csr {
   size_t smem_bytes = 0;    // dynamic smem of the staged kernels
   int grid = 0;             // persistent grid (multiple of the SM count)
   int ctas_per_sm = 0;      // resident CTAs per SM the ring was sized for
+  // Dictionary encoding (built by plan() when the operator has at most kDictMax distinct (column - row, value)
+  // pairs, as stencil and structured-grid operators do).  The staged SpMV and the persistent CG kernel then stream
+  // one code byte per nonzero instead of colind + val; every other kernel keeps reading the CSR arrays above.
+  uint8_t* code = nullptr;  // nnz (+ pad): index into the dictionary of each nonzero, in the stored order
+  void* dict = nullptr;     // kDictMax int32 column offsets, then kDictMax T values (sorted by offset, bit pattern)
+  int ndict = 0;            // dictionary entries in use; 0: no encoding
+  int dict_stages = 0;      // ring depth of the encoded pipeline (same grid and CTAs per SM as the CSR plan)
+  size_t dict_smem_bytes = 0;
 };
+constexpr int kDictMax = 256;
 
 template <class T> void csr_upload(Ctx& c, Csr<T>& A, int n, long long nnz, const void* rowptr, const void* colind,
                                    const T* val, int index_base, int index_bytes, bool on_device);

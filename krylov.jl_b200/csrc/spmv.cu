@@ -5,6 +5,8 @@
 #include "kb_internal.h"
 #include "spmv_tiles.cuh"
 
+#include <algorithm>
+#include <type_traits>
 #include <vector>
 
 namespace kb {
@@ -87,7 +89,7 @@ void csr_upload(Ctx& c, Csr<T>& A, int n, long long nnz, const void* rowptr, con
 }
 
 template <class T> void csr_free(Csr<T>& A) {
-  dev_free(A.rowptr); dev_free(A.colind); dev_free(A.val);
+  dev_free(A.rowptr); dev_free(A.colind); dev_free(A.val); dev_free(A.code); dev_free(A.dict);
   A = Csr<T>();
 }
 
@@ -122,6 +124,187 @@ __global__ void plan_kernel(int n, int ntiles, const int* __restrict__ rowptr,
   atomicMax(&out[4], mc);
   if (uns) atomicExch(&out[2], 1);
   if (neg) atomicExch(&out[5], 1);
+}
+
+// ---------------------------------------------------------------------------
+// Dictionary encoding: every nonzero k of row i is the pair (colind[k] - i, bit pattern of val[k]).  Operators with at
+// most kDictMax distinct pairs (stencils, structured grids) are stored once more as one code byte per nonzero; the
+// values are compared by bit pattern, so 0.0 / -0.0 stay distinct and decoding is exact.
+//   pass 1 (dict_collect_kernel): each warp keeps a table of the pairs it has seen (de-duplicated with
+//           __match_any_sync), the warps of a CTA merge theirs, dict_merge_kernel merges the CTAs' tables.  Any table
+//           outgrowing kDictMax raises `overflow`, which every warp polls: a general matrix is rejected after a
+//           fraction of one pass.
+//   host:   sort the pairs by (offset, bits) -- code numbering independent of the scheduling, encoding deterministic.
+//   pass 2 (dict_encode_kernel): binary search of each pair in the sorted table.
+// ---------------------------------------------------------------------------
+template <class T> using DictBits = typename std::conditional<sizeof(T) == 8, unsigned long long, unsigned>::type;
+__device__ __forceinline__ unsigned long long dict_bits(double v) { return (unsigned long long)__double_as_longlong(v); }
+__device__ __forceinline__ unsigned dict_bits(float v) { return __float_as_uint(v); }
+
+// Lanes with `have` add (off, bits) to the warp's table [0, cnt) unless it is there.  Returns the new count (warp-
+// uniform); entries past kDictMax are counted but not stored.
+template <class B>
+__device__ __forceinline__ int dict_warp_insert(int* toff, B* tbits, int cnt, bool have, int off, B bits) {
+  const int lane = threadIdx.x & 31;
+  bool need = have;
+  for (int e = 0; need && e < cnt; e++) need = !(toff[e] == off && tbits[e] == bits);
+  const unsigned needm = __ballot_sync(0xffffffffu, need);
+  if (!needm) return cnt;
+  const unsigned same = __match_any_sync(0xffffffffu, off) & __match_any_sync(0xffffffffu, bits) & needm;
+  const bool lead = need && (__ffs(same) - 1 == lane);
+  const unsigned leads = __ballot_sync(0xffffffffu, lead);
+  const int slot = cnt + __popc(leads & ((1u << lane) - 1u));
+  if (lead && slot < kDictMax) { toff[slot] = off; tbits[slot] = bits; }
+  __syncwarp();
+  return cnt + __popc(leads);
+}
+
+constexpr int kDictWarps = 8;
+
+template <class T>
+__global__ void __launch_bounds__(kDictWarps * 32) dict_collect_kernel(int n, const int* __restrict__ rowptr, const int* __restrict__ colind,
+                                                                     const T* __restrict__ val, int* cta_off, DictBits<T>* cta_bits,
+                                                                     int* cta_cnt, int* overflow) {
+  typedef DictBits<T> B;
+  __shared__ int soff[kDictWarps][kDictMax];
+  __shared__ B sbits[kDictWarps][kDictMax];
+  __shared__ int scnt[kDictWarps];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int stride = gridDim.x * kDictWarps * 32;
+  int cnt = 0;
+  for (int base = (blockIdx.x * kDictWarps + warp) * 32; base < n && cnt <= kDictMax; base += stride) {
+    if (__any_sync(0xffffffffu, *(volatile int*)overflow != 0)) break;     // another warp has already seen too many
+    const int row = base + lane;
+    int kb = 0, ke = 0;
+    if (row < n) { kb = rowptr[row]; ke = rowptr[row + 1]; }
+    const int len = __reduce_max_sync(0xffffffffu, (unsigned)(ke - kb));
+    for (int j = 0; j < len && cnt <= kDictMax; j++) {
+      const bool have = kb + j < ke;
+      const int off = have ? colind[kb + j] - row : 0;
+      const B bits = have ? dict_bits(val[kb + j]) : B(0);
+      cnt = dict_warp_insert<B>(soff[warp], sbits[warp], cnt, have, off, bits);
+    }
+  }
+  if (lane == 0) { scnt[warp] = cnt; if (cnt > kDictMax) atomicExch(overflow, 1); }
+  __syncthreads();
+  if (warp != 0) return;
+  for (int w = 1; w < kDictWarps && cnt <= kDictMax; w++) {
+    const int m = min(scnt[w], kDictMax);
+    for (int e0 = 0; e0 < m && cnt <= kDictMax; e0 += 32) {
+      const int e = e0 + lane;
+      cnt = dict_warp_insert<B>(soff[0], sbits[0], cnt, e < m, e < m ? soff[w][e] : 0, e < m ? sbits[w][e] : B(0));
+    }
+  }
+  if (cnt > kDictMax) { if (lane == 0) atomicExch(overflow, 1); }
+  for (int e = lane; e < min(cnt, kDictMax); e += 32) {
+    cta_off[blockIdx.x * kDictMax + e] = soff[0][e];
+    cta_bits[blockIdx.x * kDictMax + e] = sbits[0][e];
+  }
+  if (lane == 0) cta_cnt[blockIdx.x] = cnt;
+}
+
+// One warp: merge the CTAs' tables into out_* ([0] of out_cnt: number of pairs, kDictMax + 1 when there are more).
+template <class B>
+__global__ void dict_merge_kernel(int ncta, const int* cta_off, const B* cta_bits, const int* cta_cnt, const int* overflow,
+                                  int* out_off, B* out_bits, int* out_cnt) {
+  __shared__ int soff[kDictMax];
+  __shared__ B sbits[kDictMax];
+  const int lane = threadIdx.x;
+  int cnt = *(volatile const int*)overflow ? kDictMax + 1 : 0;
+  for (int b = 0; b < ncta && cnt <= kDictMax; b++) {
+    const int m = cta_cnt[b];
+    for (int e0 = 0; e0 < m && cnt <= kDictMax; e0 += 32) {
+      const int e = e0 + lane;
+      const bool have = e < m;
+      cnt = dict_warp_insert<B>(soff, sbits, cnt, have, have ? cta_off[b * kDictMax + e] : 0, have ? cta_bits[b * kDictMax + e] : B(0));
+    }
+  }
+  for (int e = lane; e < min(cnt, kDictMax); e += 32) { out_off[e] = soff[e]; out_bits[e] = sbits[e]; }
+  if (lane == 0) *out_cnt = min(cnt, kDictMax + 1);
+}
+
+// code[k] = position of nonzero k's pair in the sorted dictionary (kDictMax offsets, then kDictMax values).
+template <class T>
+__global__ void __launch_bounds__(kBlock) dict_encode_kernel(int n, const int* __restrict__ rowptr, const int* __restrict__ colind,
+                                                            const T* __restrict__ val, const void* dict, int ndict,
+                                                            uint8_t* __restrict__ code, int* missing) {
+  typedef DictBits<T> B;
+  __shared__ int soff[kDictMax];
+  __shared__ B sbits[kDictMax];
+  for (int e = threadIdx.x; e < ndict; e += blockDim.x) {
+    soff[e] = reinterpret_cast<const int*>(dict)[e];
+    sbits[e] = dict_bits(reinterpret_cast<const T*>(reinterpret_cast<const int*>(dict) + kDictMax)[e]);
+  }
+  __syncthreads();
+  const int stride = gridDim.x * blockDim.x;
+  for (int row = blockIdx.x * blockDim.x + threadIdx.x; row < n; row += stride) {
+    const int ke = rowptr[row + 1];
+    for (int k = rowptr[row]; k < ke; k++) {
+      const int off = colind[k] - row;
+      const B bits = dict_bits(val[k]);
+      int lo = 0, hi = ndict;                 // first entry >= (off, bits)
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (soff[mid] < off || (soff[mid] == off && sbits[mid] < bits)) lo = mid + 1;
+        else hi = mid;
+      }
+      if (lo < ndict && soff[lo] == off && sbits[lo] == bits) code[k] = (uint8_t)lo;
+      else atomicExch(missing, 1);
+    }
+  }
+}
+
+// Builds A.code / A.dict / A.ndict when the operator has at most kDictMax distinct pairs (else leaves ndict = 0).
+template <class T> static void csr_dict_build(Ctx& c, Csr<T>& A) {
+  typedef DictBits<T> B;
+  const int ncta = sm_count() * 2;
+  char* tmp = nullptr;
+  const size_t tab = (size_t)ncta * kDictMax;
+  const size_t bytes = tab * (sizeof(int) + sizeof(B)) + (size_t)ncta * sizeof(int) + kDictMax * (sizeof(int) + sizeof(B)) + 4 * sizeof(int);
+  KB_CUDA(cudaMalloc((void**)&tmp, bytes));
+  B* cta_bits = (B*)tmp;
+  B* out_bits = cta_bits + tab;
+  int* cta_off = (int*)(out_bits + kDictMax);
+  int* out_off = cta_off + tab;
+  int* cta_cnt = out_off + kDictMax;
+  int* flags = cta_cnt + ncta;                 // [0] overflow  [1] pairs found  [2] pair missing from the table
+  int h[3] = {0, 0, 0};
+  std::vector<int> hoff(kDictMax);
+  std::vector<B> hbits(kDictMax);
+  try {
+    KB_CUDA(cudaMemsetAsync(flags, 0, 4 * sizeof(int), c.stream));
+    dict_collect_kernel<T><<<ncta, kDictWarps * 32, 0, c.stream>>>(A.n, A.rowptr, A.colind, A.val, cta_off, cta_bits, cta_cnt, flags);
+    dict_merge_kernel<B><<<1, 32, 0, c.stream>>>(ncta, cta_off, cta_bits, cta_cnt, flags, out_off, out_bits, flags + 1);
+    KB_CUDA(cudaGetLastError());
+    KB_CUDA(cudaMemcpyAsync(h, flags, 2 * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
+    KB_CUDA(cudaMemcpyAsync(hoff.data(), out_off, kDictMax * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
+    KB_CUDA(cudaMemcpyAsync(hbits.data(), out_bits, kDictMax * sizeof(B), cudaMemcpyDeviceToHost, c.stream));
+    c.sync();
+    const int nd = h[1];
+    if (nd >= 1 && nd <= kDictMax) {
+      std::vector<std::pair<int, B>> pairs(nd);
+      for (int e = 0; e < nd; e++) pairs[e] = {hoff[e], hbits[e]};
+      std::sort(pairs.begin(), pairs.end());
+      std::vector<char> hd(TileLayout<T, true>::dict_bytes(), 0);
+      int* doff = (int*)hd.data();
+      T* dval = (T*)(doff + kDictMax);
+      for (int e = 0; e < nd; e++) { doff[e] = pairs[e].first; memcpy(&dval[e], &pairs[e].second, sizeof(T)); }
+      A.dict = dev_alloc<char>(hd.size());
+      A.code = reinterpret_cast<uint8_t*>(dev_alloc<char>((size_t)A.nnz + 64));       // the bulk copies read whole 16-B granules past nnz
+      KB_CUDA(cudaMemcpyAsync(A.dict, hd.data(), hd.size(), cudaMemcpyHostToDevice, c.stream));
+      KB_CUDA(cudaMemsetAsync(A.code + A.nnz, 0, 64, c.stream));
+      dict_encode_kernel<T><<<sm_count() * 4, kBlock, 0, c.stream>>>(A.n, A.rowptr, A.colind, A.val, A.dict, nd, A.code, flags + 2);
+      KB_CUDA(cudaGetLastError());
+      KB_CUDA(cudaMemcpyAsync(&h[2], flags + 2, sizeof(int), cudaMemcpyDeviceToHost, c.stream));
+      c.sync();
+      if (h[2]) throw std::runtime_error("CSR operator: dictionary encoding lost a (column offset, value) pair");
+      A.ndict = nd;
+    }
+  } catch (...) {
+    cudaFree(tmp);
+    throw;
+  }
+  cudaFree(tmp);
 }
 
 template <class T> void csr_plan(Ctx& c, Csr<T>& A) {
@@ -171,6 +354,7 @@ template <class T> void csr_plan(Ctx& c, Csr<T>& A) {
     if (L.total_bytes(s) <= two_cta) { A.tma_ok = true; A.stages = s; per_sm = 2; }
   for (int s = 4; s >= 2 && !A.tma_ok; s--)
     if (L.total_bytes(s) <= one_cta) { A.tma_ok = true; A.stages = s; per_sm = 1; }
+  const bool default_plan = A.tma_ok && per_sm == 3 && !(es && ec);
   if (A.tma_ok) {
     A.smem_bytes = L.total_bytes(A.stages);
     int g = sm_count() * per_sm;
@@ -178,6 +362,21 @@ template <class T> void csr_plan(Ctx& c, Csr<T>& A) {
     A.ctas_per_sm = per_sm;
   } else {
     A.stages = 0; A.smem_bytes = 0; A.grid = 0;
+  }
+  // Dictionary codes for the default ring (3 CTAs/SM, the same grid: the encoded kernels reduce in the same order).
+  // A stage shrinks from ~23 KB to ~3 KB (cfg2), so the encoded ring is 4 deep -- the producer runs further ahead
+  // across the persistent kernel's grid barriers -- and what the CTAs leave of the 228 KB goes to L1 for the gathers.
+  // KB200_CSR_DICT=0 keeps the CSR stream (A/B runs and tests on one build).
+  const char* ed = getenv("KB200_CSR_DICT");
+  if (default_plan && A.nnz > 0 && !(ed && atoi(ed) == 0)) {
+    const TileLayout<T, true> Ld{A.tile_cap};
+    for (int s = 4; s >= 2 && !A.dict_stages; s--)
+      if (Ld.total_bytes(s) * 3 <= 226 * 1024) A.dict_stages = s;
+    if (A.dict_stages) {
+      csr_dict_build<T>(c, A);
+      if (A.ndict) A.dict_smem_bytes = Ld.total_bytes(A.dict_stages);
+      else A.dict_stages = 0;
+    }
   }
 }
 
@@ -205,13 +404,13 @@ __global__ void __launch_bounds__(kBlock) spmv_rows_kernel(Csr<T> A, G xg, T* __
   }
 }
 
-template <class T, bool DOT, class G>
+template <class T, bool DOT, class G, bool DICT>
 __global__ void __launch_bounds__(kTileThreads, 3) spmv_tma_kernel(Csr<T> A, G xg, T* __restrict__ y, T* part,
                                                                 unsigned* ticket, T* out) {
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ T sm[32];
   T dacc = T(0);
-  spmv_tiles_run<T>(
+  spmv_tiles_run<T, DICT>(
       A, smem, xg, [&](int row) { return DOT ? __ldg(&xg.x[row]) : T(0); },
       [&](int row, T acc, T xr) {
         y[row] = acc;
@@ -229,12 +428,18 @@ static void spmv_launch_g(Ctx& c, const Csr<T>& A, G xg, T* y, int slot, int var
   const bool staged = variant == 2 || (variant == 0 && A.tma_ok);
   if (staged) {
     if (!A.tma_ok) throw std::runtime_error("TMA-staged SpMV requested but the tile plan does not fit shared memory");
-    ensure_dyn_smem((const void*)spmv_tma_kernel<T, DOT, G>, 220 * 1024);
+    // the dictionary-encoded stream when the operator has one (single GPU: the row-partitioned gather stays on CSR)
+    auto kern = spmv_tma_kernel<T, DOT, G, false>;
+    size_t smem = A.smem_bytes;
+    if constexpr (std::is_same<G, XPlain<T>>::value) {
+      if (A.ndict > 0) { kern = spmv_tma_kernel<T, DOT, G, true>; smem = A.dict_smem_bytes; }
+    }
+    ensure_dyn_smem((const void*)kern, 220 * 1024);
     int occ = 0;   // persistent grid = what is really co-resident (never more than one wave)
-    KB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, spmv_tma_kernel<T, DOT, G>, kTileThreads, A.smem_bytes));
+    KB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kTileThreads, smem));
     if (occ < 1) throw std::runtime_error("spmv_tma_kernel does not fit on an SM with the planned shared-memory ring");
     const int grid = std::min(std::min(occ, A.ctas_per_sm) * sm_count(), std::max(1, A.ntiles));
-    spmv_tma_kernel<T, DOT, G><<<grid, kTileThreads, A.smem_bytes, c.stream>>>(A, xg, y, (T*)c.partials, c.tickets + 1, out);
+    kern<<<grid, kTileThreads, smem, c.stream>>>(A, xg, y, (T*)c.partials, c.tickets + 1, out);
   } else {
     const int grid = stream_grid(A.n, 1, 8);
     spmv_rows_kernel<T, DOT, G><<<grid, kBlock, 0, c.stream>>>(A, xg, y, (T*)c.partials, c.tickets + 1, out);

@@ -83,6 +83,7 @@ SIGNATURES = {
     "krylov_b200_set_operator_csr": (_I, [_P, _I, _LL, _P, _P, _P, _I, _I, _I]),
     "krylov_b200_share_operator": (_I, [_P, _P]),
     "krylov_b200_attach_csr": (_I, [_P, _P]),
+    "krylov_b200_operator_encoding": (_I, [_P]),
     "krylov_b200_set_preconditioner_diag": (_I, [_P, _I, _P, _I]),
     "krylov_b200_set_preconditioner_blockdiag": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_int]),
     "krylov_b200_default_options": (KrylovB200Options, []),
